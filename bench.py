@@ -3,6 +3,7 @@
 
   python bench.py --gpus N --steps K --warmup W            # this engine   (N>1: launched under torchrun, one rank per GPU)
   python bench.py --impl reference --gpus N --steps K ...   # the reference's own CPU implementation on the host cores
+  python bench.py ... --dump-outputs DIR                    # also write the PCM of the last timed step to DIR/*.npy
 
 Metric (BASELINE.json): synthesized 16 kHz samples/s over batched independent streams.
 A "step" = one pass of the hot path over one batch of synthetic feature frames:
@@ -18,6 +19,11 @@ A "step" = one pass of the hot path over one batch of synthetic feature frames:
            SMs, lpcnet_b200/csrc/microbench.cu).  Because one MMA fetch serves 16 streams the algorithmic figure may exceed the
            physical one; the physical evidence (ncu LSU-pipe %) is quoted beside it.  `sparse_gemv_frac` is the north star's
            own measure (GRU_A weights + indices only).  HBM traffic per sample (ncu) vs the 2.5 B algorithmic is reported too.
+`--dump-outputs DIR`: after the timed steps, the PCM the last step of each timed leg returned, as float32 [streams][samples]:
+           DIR/pcm.npy (`value` leg, read back from HBM) and DIR/pcm_e2e.npy (`e2e` leg, the host buffer the call filled), with
+           DIR/streams.npy, the stream index of every row.  Above DUMP_LIMIT bytes in all, the same seeded sample of streams is
+           kept from both.  The inputs and the number of steps before the last one depend only on the arguments, so two builds
+           run with the same arguments can be compared array for array.
 `cpu_baseline`: the untouched reference compiled by oracle/Makefile (oracle/_ref, timing builds T / TB = -Ofast AVX2/FMA,
            int8 / float) on this box's host cores, one independent stream per usable hardware thread (affinity mask and
            cgroup quota respected), state creation + model load OUTSIDE the timer; plus the 1-core figure.  Falls back to
@@ -44,6 +50,7 @@ STREAMS_PER_GPU = 4096
 FRAMES = 10               # frames per step (1600 samples per stream per step)
 LPC_GAMMA = 0.9
 METRIC = "16 kHz samples/sec (batched independent streams), whole job"
+DUMP_LIMIT = 64 * 10 ** 6  # bytes written by --dump-outputs, all files together
 UNIT = "samples/s"
 
 
@@ -149,6 +156,25 @@ def measured_peaks():
     return 6650.0, "fallback (B200_PROFILING.md)"
 
 
+def dump_rows(rows, cols, narrays):
+    """Stream indices --dump-outputs writes: all of them, or a fixed seeded sample when narrays float32 arrays of
+    [rows][cols] and the index list would exceed DUMP_LIMIT."""
+    keep = (DUMP_LIMIT - 8 * rows - 4096) // (4 * cols * narrays)        # 4096: the .npy headers
+    if keep < 1:
+        raise SystemExit("bench: --dump-outputs: one stream's output alone exceeds %d bytes" % DUMP_LIMIT)
+    if keep >= rows:
+        return np.arange(rows)
+    return np.sort(np.random.default_rng(0).choice(rows, keep, replace=False))
+
+
+def dump_outputs(out_dir, rows, arrays):
+    """arrays: name -> int16 PCM [streams][samples]; writes out_dir/<name>.npy (float32, exact for int16) and out_dir/streams.npy."""
+    os.makedirs(out_dir, exist_ok=True)
+    np.save(os.path.join(out_dir, "streams.npy"), rows.astype(np.float64))
+    for name, a in arrays.items():
+        np.save(os.path.join(out_dir, name + ".npy"), a[rows].astype(np.float32))
+
+
 # ---------------------------------------------------------------------------------------------------------------------
 CPU_WORK = {  # workload -> (reference timing build, blob kind, description)
     "config3_int8": ("T", "int8", "lpcnet_synthesize, int8 AVX2 path (-Ofast -mavx2 -mfma)"),
@@ -241,7 +267,10 @@ def main():
     ap.add_argument("--streams", type=int, default=0, help="streams per GPU (default: 4096 / 256 / 1024 by workload)")
     ap.add_argument("--frames", type=int, default=FRAMES, help="frames per step")
     ap.add_argument("--no-cpu-baseline", action="store_true")
+    ap.add_argument("--dump-outputs", metavar="DIR", help="write the PCM of the last timed step of both legs to DIR/*.npy")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
     args.warmup = max(args.warmup, 3) if args.impl == "engine" else args.warmup
 
     rank = int(os.environ.get("RANK", "0"))
@@ -260,8 +289,6 @@ def main():
 
     import helpers as H
     import lpcnet_b200
-    from lpcnet_b200 import build
-    build.build()
     if lpcnet_b200.device_count() <= 0:
         raise SystemExit("bench: no CUDA device; this engine has no CPU fallback")
     L = lpcnet_b200.lib()
@@ -279,6 +306,9 @@ def main():
     else:
         feats = features_for(n, F, first_stream=n * rank)           # distinct per stream (and per rank)
     fbytes, pbytes = feats.nbytes, n * F * 160 * 2
+    dump = rank == 0 and args.dump_outputs
+    if dump:
+        rows = dump_rows(world * n, F * 160, 2)
     L.lpcnet_b200_set_device(local)
     d_feat = L.lpcnet_b200_device_alloc(fbytes)
     d_pcm = L.lpcnet_b200_device_alloc(pbytes)
@@ -351,6 +381,9 @@ def main():
     wall = time.time() - wall0
     clk = clocks.stop()
     dev_s = sum(step_ms) * 1e-3
+    if dump:                                                 # the last step's PCM: in the job's gather buffer when N > 1
+        pcm_dev = np.empty((world * n, F * 160), np.int16)
+        L.lpcnet_b200_memcpy_d2h(pcm_dev.ctypes.data, d_gather if dist is not None else d_pcm, pbytes * world)
     # ---------------- timed: end-to-end through the host-pointer C-ABI ----------------
     for _ in range(2):
         step_e2e()
@@ -363,6 +396,8 @@ def main():
         e2e_ms.append(batch.timer_stop())
     barrier()
     e2e_s = sum(e2e_ms) * 1e-3
+    if dump and dist is None:
+        pcm_e2e = np.ctypeslib.as_array(ctypes.cast(h_pcm_p, ctypes.POINTER(ctypes.c_int16)), shape=(n, F * 160)).copy()
 
     if dist is not None:
         import torch
@@ -379,6 +414,7 @@ def main():
         if rank == 0:
             full = np.empty((world * n, F * 160), np.int16)
             L.lpcnet_b200_memcpy_d2h(full.ctypes.data, d_gather, pbytes * world)
+            pcm_e2e = full
             gather_ok = all(hashlib.sha256(full[r * n:(r + 1) * n].tobytes()).hexdigest() == digs[r] for r in range(world))
             if os.environ.get("LPCNET_B200_BENCH_DIRECT_SINK"):
                 gather_ok = None                                  # (experiment: the e2e leg does not write the gather buffer)
@@ -388,6 +424,8 @@ def main():
     else:
         gather_ms = None
 
+    if dump:
+        dump_outputs(args.dump_outputs, rows, {"pcm": pcm_dev, "pcm_e2e": pcm_e2e})
     if rank == 0:
         samples_step = world * n * F * 160
         value = samples_step * args.steps / dev_s

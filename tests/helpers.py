@@ -201,6 +201,33 @@ def stream_digests(pcm):
     return np.array([int.from_bytes(hashlib.sha256(np.ascontiguousarray(r).tobytes()).digest()[:8], "little") for r in pcm], dtype=np.uint64)
 
 
+def digests(a):
+    """stream_digests of every a[i], whatever its shape: one digest per stream, frame or packet."""
+    return stream_digests(np.reshape(a, (len(a), -1)))
+
+
+@functools.lru_cache(None)
+def ref_checks():
+    """What the compiled reference returned for the inputs of the tests that compare with it (tests/golden/make_golden_ref_checks.py)."""
+    return dict(np.load(os.path.join(GOLDEN, "ref_checks.npz")))
+
+
+def assert_ref_digests(got, key, what):
+    """digests(got) against the stored digests of the reference's output; a failure names the rows that differ."""
+    want = ref_checks()[key]
+    bad = np.nonzero(digests(got) != want)[0]
+    assert bad.size == 0, "%s: %d of %d rows differ from the reference, first: %s" % (what, bad.size, len(want), bad[:16].tolist())
+
+
+def activation_test_inputs():
+    """(x, v): float32 inputs of the tanh / sigmoid and of the lin2ulaw comparison."""
+    rng = np.random.default_rng(3)
+    x = np.concatenate([rng.normal(0, 3, 20000), rng.uniform(-12, 12, 20000), [0.0, -0.0, 1e-8, 50.0, -50.0]]).astype(np.float32)
+    x = x[: x.size // 8 * 8]
+    v = np.concatenate([rng.normal(0, 3000, 20000), rng.uniform(-40000, 40000, 5000), [0.0, 32767.0, -32768.0]]).astype(np.float32)
+    return x, v
+
+
 # ---- the analysis side (SURVEY 8f N2): the compiled reference's encoder entry points, one fresh state per stream ----
 def ref_features(pcm, build="A"):
     """pcm [n][T*160] int16 (or float32) -> features [n][T][36] via lpcnet_compute_single_frame_features(_float)."""

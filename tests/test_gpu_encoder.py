@@ -1,8 +1,8 @@
 """GPU tests (-m gpu) of the analysis side (SURVEY 8f N2): batched feature extraction and the 1.6 kb/s encoder
 (lpcnet_b200_enc_*, csrc/enc_kernels.cu) against the reference's lpcnet_compute_single_frame_features / lpcnet_encode /
 lpcnet_compute_features (src/lpcnet_enc.c).  The bar is the same as on the synthesis side: every feature float and every packet
-byte equal to the reference's (goldens produced by the compiled reference, tests/golden/make_golden_enc.py; where the compiled
-reference itself travelled, oracle/_ref, also fresh inputs).  Floats are compared as bit patterns."""
+byte equal to the reference's (goldens produced by the compiled reference, tests/golden/make_golden_enc.py, and digests of its
+output on fresh inputs, tests/golden/make_golden_ref_checks.py).  Floats are compared as bit patterns."""
 import ctypes
 import os
 import subprocess
@@ -158,18 +158,18 @@ def test_fresh_inputs_against_the_oracle_port(eng):
     assert_same_floats(f4, H.oracle_encode(pcm, features4=True), "features4 vs oracle port")
 
 
-@pytest.mark.skipif(not H.have_ref("A"), reason="compiled reference (oracle/_ref) did not travel")
 def test_fresh_inputs_against_the_compiled_reference(eng):
-    """96 other streams x 60 frames (15 packets): features and packets equal the compiled reference run on this host."""
+    """96 other streams x 60 frames (15 packets): features and packets equal what the compiled reference returned, stream by stream."""
     n, T = 96, 60
     pcm = make_pcm_batch(range(100, 100 + n), T)
+    H.assert_ref_digests(pcm, "gpu_enc_pcm", "test inputs")
     e = eng.EncBatch(n, codebooks=H.codebooks())
     f = e.compute_features(pcm)
     e.reset()
     pk = e.encode(pcm)
     e.close()
-    assert_same_floats(f, H.ref_features(pcm), "features, fresh streams")
-    np.testing.assert_array_equal(pk, H.ref_encode(pcm))
+    H.assert_ref_digests(f, "gpu_enc_features", "features, fresh streams")
+    H.assert_ref_digests(pk, "gpu_enc_packets", "packets, fresh streams")
 
 
 @pytest.mark.skipif(not os.path.exists(os.path.join(H.ORACLE, "_ref", "lpcnet_demo_b200")), reason="reference CLI linked against liblpcnet_b200.so not built")

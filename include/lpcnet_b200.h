@@ -262,7 +262,10 @@ LPCNET_EXPORT int lpcnet_b200_batch_get_state(LPCNetB200Batch *b, int s, float *
 LPCNET_EXPORT int lpcnet_b200_debug_frame_network(LPCNetB200Batch *b, const float *features, int nframes,
                                                   int feature_stride, float *ga, float *gb, float *lpc);
 /* Test hook (host only, no CUDA): build the per-sample kernel's shared-memory image for a blob.  Returns the
- * image size or <0; layout[24] receives the offsets documented in lpcnet_b200/csrc/batch_api.cu. */
+ * image size or <0; layout[24] receives the offsets documented in lpcnet_b200/csrc/batch_api.cu.  layout[21] is 1 when
+ * the model's range bound lets the int8 kernel round the GRU_A accumulators without the conversion unit (acc_init_t<true>,
+ * lpcnet_b200/csrc/devmath.cuh), 0 when it converts with cvt (always 0 for float blobs); layout[22] is 1 for a float blob, whose
+ * image and offsets are those of the lane==stream float kernel. */
 LPCNET_EXPORT int lpcnet_b200_debug_image(const unsigned char *blob, int len, unsigned char *out, size_t cap,
                                           uint32_t *layout);
 

@@ -936,17 +936,25 @@ int lpcnet_b200_debug_frame_network(LPCNetB200Batch *b, const float *features, i
 }
 
 // Test hook (host only, no CUDA): the shared-memory image and its run-time layout words
-// layout[8] = {wA, metaA, wB, metaB, image_bytes, total_bytes, nblkA_padded, nblkB_padded}; also returns sm_image in layout[8].
+// layout = {wA, metaA, wB, metaB, image_bytes, total_bytes, nblkA_padded, nblkB_padded, sm_image, para, dira, grpa, dirb,
+// wbrec, parb, fcw, compute warps, groups per compute warp, dual_fc rows in shared memory, K parts of GRU_B, na, fast_cvt, is_float}.
+// Offsets 9..15 are relative to sm_image and belong to the kernel that reads the image: the int8 kernel, or for float blobs the
+// lane==stream float kernel (which keeps no dual_fc rows in shared memory: fcw = ~0, rows = 0).
 int lpcnet_b200_debug_image(const unsigned char *blob, int len, unsigned char *out, size_t cap, uint32_t *layout)
 {
-    SmemLayout L; Geom G;
-    int r = debug_build_image(blob, len, out, cap, &L, &G);
+    SmemLayout L; Geom G; int fast_cvt = 0, is_float = 0;
+    int r = debug_build_image(blob, len, out, cap, &L, &G, &fast_cvt, &is_float);
     if (r < 0) return r;
     layout[0] = L.wA; layout[1] = L.metaA; layout[2] = L.wB; layout[3] = L.metaB; layout[4] = L.image_bytes; layout[5] = L.total_bytes;
     layout[6] = L.nblkA_padded; layout[7] = L.nblkB_padded; layout[8] = L.sm_image;
-    layout[9] = G.im_para; layout[10] = G.im_dira; layout[11] = G.im_grpa; layout[12] = G.im_dirb; layout[13] = G.im_wbrec; layout[14] = G.im_parb;
-    layout[15] = G.im_fcw; layout[16] = NWC; layout[17] = G.gpw; layout[18] = *reinterpret_cast<const uint32_t *>(out + G.im_fcwn); layout[19] = KPARTS;
-    layout[20] = G.na;
+    if (is_float) {
+        layout[9] = G.fi_para; layout[10] = G.fi_dira; layout[11] = G.fi_grpa; layout[12] = G.fi_dirb; layout[13] = L.wBrecF - L.sm_image; layout[14] = G.fi_parb;
+        layout[15] = 0xFFFFFFFFu; layout[16] = F_NWC; layout[17] = G.f_gpw; layout[18] = 0; layout[19] = F_KPARTS;
+    } else {
+        layout[9] = G.im_para; layout[10] = G.im_dira; layout[11] = G.im_grpa; layout[12] = G.im_dirb; layout[13] = G.im_wbrec; layout[14] = G.im_parb;
+        layout[15] = G.im_fcw; layout[16] = NWC; layout[17] = G.gpw; layout[18] = *reinterpret_cast<const uint32_t *>(out + G.im_fcwn); layout[19] = KPARTS;
+    }
+    layout[20] = G.na; layout[21] = (uint32_t)fast_cvt; layout[22] = (uint32_t)is_float;
     return r;
 }
 

@@ -367,7 +367,7 @@ inline size_t condA_frame_floats(bool is_float, size_t n, int na) { return is_fl
 // ---- host-side API of the internal modules ----
 int model_load(DeviceModel *m, const unsigned char *blob, int len, const ModelConfig *cfg);   // 0 / -1 (sets error); cfg NULL = blob metadata / defaults
 void model_free(DeviceModel *m);
-int debug_build_image(const unsigned char *blob, int len, unsigned char *out, size_t cap, SmemLayout *L, Geom *g);
+int debug_build_image(const unsigned char *blob, int len, unsigned char *out, size_t cap, SmemLayout *L, Geom *g, int *fast_cvt, int *is_float);
 int debug_build_image_n(const unsigned char *blob, int len, unsigned char *out, size_t cap, SmemLayout *L, Geom *g);
 void set_error(const char *fmt, ...);
 

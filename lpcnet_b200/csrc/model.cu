@@ -525,11 +525,11 @@ static int build_host_model(DeviceModel *m, HostModel &hm, const unsigned char *
 }
 
 // Test hook (no CUDA needed): build the shared-memory image on the host and hand it out.
-int debug_build_image(const unsigned char *blob, int len, unsigned char *out, size_t cap, SmemLayout *L, Geom *g)
+int debug_build_image(const unsigned char *blob, int len, unsigned char *out, size_t cap, SmemLayout *L, Geom *g, int *fast_cvt, int *is_float)
 {
     DeviceModel m; HostModel hm;
     if (build_host_model(&m, hm, blob, len, nullptr) != 0) return -1;
-    *L = m.L; *g = make_geom(m.na);
+    *L = m.L; *g = make_geom(m.na); *fast_cvt = m.fast_cvt; *is_float = m.is_float;
     if (hm.img.size() > cap) { set_error("debug image: buffer too small"); return -1; }
     memcpy(out, hm.img.data(), hm.img.size());
     return (int)hm.img.size();

@@ -100,13 +100,18 @@ def _sparse_pack(A, have_diag):
                 idx=np.array(idx, dtype=np.int32), AQ=AQ)
 
 
-def make_model(seed=1234, na=None, variant=""):
+def make_model(seed=1234, na=None, variant="", knobs=None):
     """Returns (arrays_common, arrays_int8, arrays_float): ordered lists of (name, type, ndarray).
     na      : GRU_A units (default 384; other sizes are the `--grua-size` models of training_tf2/train_lpcnet.py)
     variant : "" | "clamp" (sampling tree biased towards large excitation so that the output runs into the +-32767 clamp of
-              lpcnet.c:265-269) | "dense" (GRU_A block densities 10/10/30 %)"""
+              lpcnet.c:265-269) | "dense" (GRU_A block densities 10/10/30 %)
+    knobs   : hooks of the stress models (STRESS below); without them the random draws are exactly those of the regular models.
+              density (z, r, h); a_mask(k, rng, N_A) -> bool [N_A/4 col blocks][N_A/8 row groups] of gate k or None (random);
+              a_q(k, q, mask) -> int GRU_A gate matrix [in][out] after masking; b_in(q) / b_rec(q) -> GRU_B input / recurrent
+              int matrix [in][out]; diag(k, d) -> GRU_A diagonal of gate k"""
     N_A = int(na or globals()["N_A"])
-    DENSITY = (0.10, 0.10, 0.30) if variant == "dense" else globals()["DENSITY"]
+    kn = knobs or {}
+    DENSITY = kn.get("density") or ((0.10, 0.10, 0.30) if variant == "dense" else globals()["DENSITY"])
     rng = np.random.default_rng(seed)
     f32 = np.float32
     common, only8, onlyf = [], [], []
@@ -132,11 +137,15 @@ def make_model(seed=1234, na=None, variant=""):
     fl("gru_b_dense_feature_weights", rng.normal(0.0, 0.10, size=(COND, 3 * N_B)))
     fl("gru_b_dense_feature_bias", np.zeros(3 * N_B))
     qb_in = _quantized_matrix(rng, N_A, 3 * N_B, 0.09)
+    if "b_in" in kn:
+        qb_in = kn["b_in"](qb_in)
     pk = _sparse_pack(qb_in / 128.0, have_diag=False)
     only8.append(("gru_b_weights", WEIGHT_TYPE_qweight, pk["w_int8"]))
     onlyf.append(("gru_b_weights", WEIGHT_TYPE_qweight, pk["w_float"]))
     common.append(("gru_b_weights_idx", WEIGHT_TYPE_int, pk["idx"]))
     qb_rec = _quantized_matrix(rng, N_B, 3 * N_B, 0.25)
+    if "b_rec" in kn:
+        qb_rec = kn["b_rec"](qb_rec)
     # dotp layout: reshape (in/4,4,out/8,8) -> transpose (2,0,3,1) = [out/8][in/4][8][4]  (dump_lpcnet.py:58-59)
     dot = qb_rec.reshape(N_B // 4, 4, 3 * N_B // 8, 8).transpose(2, 0, 3, 1).reshape(-1)
     only8.append(("gru_b_recurrent_weights", WEIGHT_TYPE_qweight, dot.astype(np.int8)))
@@ -186,15 +195,19 @@ def make_model(seed=1234, na=None, variant=""):
     A = np.zeros((N_A, 3 * N_A))
     for k in range(3):
         nblk = (N_A // 4) * (N_A // 8)
-        keep = nblk - int(round(nblk * (1 - DENSITY[k])))
-        chosen = rng.choice(nblk, size=keep, replace=False)
-        mask = np.zeros(nblk, dtype=bool)
-        mask[chosen] = True
-        mask = mask.reshape(N_A // 4, N_A // 8)
+        mask = kn["a_mask"](k, rng, N_A) if "a_mask" in kn else None
+        if mask is None:
+            keep = nblk - int(round(nblk * (1 - DENSITY[k])))
+            chosen = rng.choice(nblk, size=keep, replace=False)
+            mask = np.zeros(nblk, dtype=bool)
+            mask[chosen] = True
+            mask = mask.reshape(N_A // 4, N_A // 8)
         q = _quantized_matrix(rng, N_A, N_A, 0.17 if k < 2 else 0.13)
         # make sure every kept block is non-empty (dump drops all-zero blocks)
         full = np.repeat(np.repeat(mask, 4, axis=0), 8, axis=1)
         q = q * full
+        if "a_q" in kn:
+            q = kn["a_q"](k, q, mask)
         for (jb, ib) in zip(*np.nonzero(mask)):
             blk = q[jb * 4:(jb + 1) * 4, ib * 8:(ib + 1) * 8]
             # the diagonal is removed by the dump; a kept block must keep an off-diagonal non-zero
@@ -209,6 +222,8 @@ def make_model(seed=1234, na=None, variant=""):
         A[:, k * N_A:(k + 1) * N_A] = q / 128.0
         # diagonal (kept outside the block structure, float, not quantised)
         d = rng.normal(0.25 if k == 2 else 0.1, 0.2, size=N_A)
+        if "diag" in kn:
+            d = kn["diag"](k, d)
         A[:, k * N_A:(k + 1) * N_A] -= np.diag(np.diag(A[:, k * N_A:(k + 1) * N_A]))
         A[:, k * N_A:(k + 1) * N_A] += np.diag(d.astype(f32).astype(np.float64))
     # pair constraint must hold after diagonal removal as well (true: removing only lowers |q|)
@@ -244,15 +259,209 @@ def write_blob(path, arrays):
 
 def _write_blob(path, arrays):
     with open(path, "wb") as f:
-        for name, typ, a in arrays:
-            raw = a.tobytes()
-            size = len(raw)
-            block = (size + 63) // 64 * 64
-            nm = name.encode()
-            assert len(nm) < 44
-            f.write(struct.pack("<4siiii44s", b"DNNw", 0, typ, size, block, nm))
-            f.write(raw)
-            f.write(b"\0" * (block - size))
+        f.write(blob_bytes(arrays))
+
+
+def blob_bytes(arrays):
+    out = []
+    for name, typ, a in arrays:
+        raw = a.tobytes()
+        size = len(raw)
+        block = (size + 63) // 64 * 64
+        nm = name.encode()
+        assert len(nm) < 44
+        out += [struct.pack("<4siiii44s", b"DNNw", 0, typ, size, block, nm), raw, b"\0" * (block - size)]
+    return b"".join(out)
+
+
+# ---------------------------------------------------------------------------------------------------------------------------------
+# Stress models (test inputs only).  The regular models above share one weight structure (random block masks at 5/5/20 %, dense GRU_B
+# input, int8 weights well inside the pair constraint, GRU_A pre-activations far below 2^22 accumulator units); a trained model has
+# uneven per-row density and weights at the WeightClip limit.  These models put the loader's and the kernels' edge cases into play:
+#   holes / holes128  empty GRU_A lists (one neuron group with all three empty, most z lists empty so that some compute warps hold
+#                     only empty z lists), lists of 1, 2, 3, 5, ... blocks; GRU_B input row groups of 0, 1, 3 and 5 blocks
+#   one_class         lists whose column blocks all share one class (pos/4) & 3: the repeated-class and empty-slot paths of the quad dealer
+#   skewed            density in four neuron groups: their compute warps fill their tensor-memory columns exactly (skewed_over: one
+#                     quad more, refused)
+#   denser            block densities 6/6/22 %: they load with fewer dual_fc rows in shared memory; denser_over, one step denser
+#                     (6.25/6.25/22.5 %, same seed), needs more shared memory than one SM has and is refused
+#   pair_edge         int8 weights -128 and same-sign pairs with |w0|+|w1| = 128 (pair_over_pos / pair_over_neg: one pair at 129, refused)
+#   cvt_fast_edge     large recurrent su-biases and diagonals on neuron group 5 (candidate gate): the range bound of the conversion-free
+#                     rounding lands just below its limit; cvt_exact_edge just above it
+STRESS_NAMES = ("holes", "holes128", "one_class", "skewed", "denser", "pair_edge", "cvt_fast_edge", "cvt_exact_edge")
+STRESS_REFUSED = ("skewed_over", "denser_over", "pair_over_pos", "pair_over_neg")
+CVT_LIMIT = 4194304.0 * 0.99           # model.cu: fast_cvt = bound < 0.99 * 2^22
+CVT_GROUP = 5                          # neuron group of the cvt models' large su-biases / diagonals
+
+
+def _list_mask(rng, n_cols, lengths, cls=None):
+    """bool [n_cols col blocks][len(lengths) row groups]: lengths[i] random column blocks for row group i (of class cls if given)."""
+    m = np.zeros((n_cols, len(lengths)), bool)
+    for i, n in enumerate(lengths):
+        cand = np.arange(n_cols) if cls is None else np.arange(cls, n_cols, 4)
+        m[rng.choice(cand, size=n, replace=False), i] = True
+    return m
+
+
+def _b_in_mask(q, lengths, rng, cls=None):
+    """Keep lengths[rg] column blocks of GRU_B input row group rg (q: int [N_A][48]); every kept block non-zero."""
+    q = q.copy()
+    keep = _list_mask(rng, q.shape[0] // 4, lengths, cls)
+    q *= np.repeat(np.repeat(keep, 4, axis=0), 8, axis=1)
+    for jb, rg in zip(*np.nonzero(keep)):
+        if not q[jb * 4:jb * 4 + 4, rg * 8:rg * 8 + 8].any():
+            q[jb * 4, rg * 8] = 1
+    return q
+
+
+def _holes_knobs(na):
+    ng, nc = na // 8, na // 4
+    cyc = [1, 2, 3, 5, 0, 4, 7, 9, 1, 6, 13, 3, 2, 5, 8, 11]
+    def a_mask(k, rng, N_A):
+        if k == 0:      # z: only every fifth group has a list (so some compute warps hold no z block at all)
+            L = [cyc[(i * 3) % len(cyc)] if i % 5 == 1 else 0 for i in range(ng)]
+        else:
+            L = [cyc[(i + 5 * k) % len(cyc)] for i in range(ng)]
+        L[0] = 0                                  # neuron group 0: z, r and h lists all empty
+        return _list_mask(rng, nc, L)
+    brng = np.random.default_rng(77)
+    return dict(a_mask=a_mask, b_in=lambda q: _b_in_mask(q, [0, 1, 3, 5, nc, nc // 2], brng))
+
+
+def _one_class_knobs(na):
+    ng, nc = na // 8, na // 4
+    def a_mask(k, rng, N_A):
+        m = np.zeros((nc, ng), bool)
+        for i in range(ng):
+            n = (1, 2, 3, 4, 5, 6, 7, 9, 12, 17, 0, 10)[(i + 4 * k) % 12] if i % 3 != 2 else 3 + (i + k) % 9
+            # two of three groups: all blocks of one class; the others: any class
+            m[:, i] = _list_mask(rng, nc, [n], cls=None if i % 3 == 2 else (i + k) % 4)[:, 0]
+        return m
+    brng = np.random.default_rng(78)
+    return dict(a_mask=a_mask, b_in=lambda q: _b_in_mask(q, [nc // 4, 5, 1, nc // 4, 2, 7], brng, cls=1))
+
+
+def _skewed_knobs(extra=0):
+    """Four heavy neuron groups (z r h = 52 + extra, 52, 48 blocks = 38 quads); 28 light ones, 16 empty.  With the GRU_B input GEMV's
+    12 quads the heavy groups' compute warps walk exactly 50 quads = 2 * (50 + 2) = 104 tensor-memory columns, all they have."""
+    ng, nc = 48, 96
+    def a_mask(k, rng, N_A):
+        L = [0] * ng
+        for i in range(ng):
+            if i in (3, 17, 30, 41):
+                L[i] = (52 + (extra if i == 3 else 0), 52, 48)[k]
+            elif i % 3 != 0:
+                L[i] = (2, 3, 5)[k] + (i % 4)
+        return _list_mask(rng, nc, L)
+    return dict(a_mask=a_mask)
+
+
+def _pair_knobs(over=0):
+    """Weights at the limits of the pair constraint in GRU_A (every gate), the GRU_B input and the GRU_B recurrent matrix.
+    over=+1 / -1: one same-sign pair of GRU_A's candidate gate at |w0|+|w1| = 129 (positive / negative)."""
+    pairs = [(-128, 0), (0, -128), (64, 64), (-64, -64), (127, 1), (-1, -127), (-128, 127), (100, 28), (-28, -100), (127, -128)]
+    def put(q, slots):
+        q = q.copy()
+        for t, (r, c) in enumerate(slots):
+            q[r, c], q[r + 1, c] = pairs[t % len(pairs)]
+        return q
+    def a_q(k, q, mask):
+        slots = []
+        for jb, ib in zip(*np.nonzero(mask)):
+            for a in (0, 2):
+                r, c = jb * 4 + a, ib * 8 + (len(slots) % 8)
+                if r != c and r + 1 != c:
+                    slots.append((r, c))
+            if len(slots) >= 40:
+                break
+        q = put(q, slots)
+        if over and k == 2:
+            r, c = slots[-1]
+            q[r, c], q[r + 1, c] = (64, 65) if over > 0 else (-128, -1)
+        return q
+    return dict(a_q=a_q,
+                b_in=lambda q: put(q, [(2 * i, (5 * i) % 48) for i in range(0, 160, 7)]),
+                b_rec=lambda q: put(q, [(2 * (i % 8), (7 * i) % 48) for i in range(20)]))
+
+
+def _cvt_knobs():
+    def diag(k, d):
+        if k == 2:
+            d = d.copy()
+            d[8 * CVT_GROUP:8 * CVT_GROUP + 8] = 40.0 + np.arange(8)
+        return d
+    return dict(diag=diag)
+
+
+def _int8_dense(w8, idx, n_in, n_out):
+    M = np.zeros((n_out, n_in), np.int64)
+    p = wp = 0
+    for rg in range(n_out // 8):
+        nb = idx[p]; p += 1
+        for _ in range(nb):
+            pos = idx[p]; p += 1
+            M[rg * 8:rg * 8 + 8, pos:pos + 4] = w8[wp:wp + 32].reshape(8, 4); wp += 32
+    return M
+
+
+def cvt_bound(common, only8):
+    """model.cu's range bound of the GRU_A accumulators (conversion-free rounding iff bound < CVT_LIMIT), in the same double arithmetic."""
+    a = {n: v for n, _, v in common + only8}
+    na = a["sparse_gru_a_recurrent_weights_diag"].size // 3
+    f64 = lambda n: a[n].astype(np.float64)
+    cmax = (np.abs(f64("gru_a_dense_feature_bias")) + np.abs(f64("gru_a_dense_feature_weights")).sum(axis=0)).max()
+    bmax = np.abs(f64("sparse_gru_a_subias")[1]).max()
+    dmax = np.abs(f64("sparse_gru_a_recurrent_weights_diag")).max()
+    emax = max(np.abs(f64("gru_a_embed_%s_weights" % s)).max() for s in ("sig", "pred", "exc"))
+    W = _int8_dense(a["sparse_gru_a_recurrent_weights"].astype(np.int64), a["sparse_gru_a_recurrent_weights_idx"], na, 3 * na)
+    smax = np.abs(W).sum(axis=1).max()
+    return (bmax + dmax + cmax + 3 * emax) * 1.01 * (128.0 * 127.0) + 255.0 * smax + 2
+
+
+def _set_cvt_bias(common, only8, ratio):
+    """Recurrent su-biases of neuron group CVT_GROUP's candidate gate (sign alternating, the largest on its first neuron) such that
+    cvt_bound = ratio * CVT_LIMIT; the float flavour's recurrent bias gets the same value plus the su-bias correction."""
+    a = {n: v for n, _, v in common}
+    sub, bias = a["sparse_gru_a_subias"], a["sparse_gru_a_bias"]
+    na = sub.shape[1] // 3
+    cols = 2 * na + 8 * CVT_GROUP + np.arange(8)
+    corr = bias[1, cols].astype(np.float64) - sub[1, cols].astype(np.float64)       # sum(AQ)/128 of those rows
+    sub[1, cols] = 0
+    rest = cvt_bound(common, only8) - 1.01 * 128.0 * 127.0 * np.abs(sub[1].astype(np.float64)).max()
+    b = (ratio * CVT_LIMIT - rest) / (1.01 * 128.0 * 127.0)
+    vals = b * (1.0 - 0.02 * np.arange(8)) * np.where(np.arange(8) % 2 == 0, 1.0, -1.0)
+    sub[1, cols] = vals.astype(np.float32)
+    bias[1, cols] = (vals + corr).astype(np.float32)
+
+
+def make_stress_model(name):
+    """(common, only8, onlyf) of a stress model (STRESS_NAMES, STRESS_REFUSED)."""
+    if name in ("holes", "holes128"):
+        na = 128 if name == "holes128" else 384
+        return make_model(2001, na=na, knobs=_holes_knobs(na))
+    if name == "one_class":
+        return make_model(2002, knobs=_one_class_knobs(384))
+    if name in ("skewed", "skewed_over"):
+        return make_model(2003, knobs=_skewed_knobs(extra=4 if name == "skewed_over" else 0))
+    if name in ("denser", "denser_over"):
+        return make_model(2004, knobs=dict(density=(0.06, 0.06, 0.22) if name == "denser" else (0.0625, 0.0625, 0.225)))
+    if name in ("pair_edge", "pair_over_pos", "pair_over_neg"):
+        return make_model(2005, knobs=_pair_knobs({"pair_edge": 0, "pair_over_pos": 1, "pair_over_neg": -1}[name]))
+    if name in ("cvt_fast_edge", "cvt_exact_edge"):
+        common, only8, onlyf = make_model(2006, knobs=_cvt_knobs())
+        _set_cvt_bias(common, only8, 0.995 if name == "cvt_fast_edge" else 1.005)
+        return common, only8, onlyf
+    raise KeyError(name)
+
+
+def stress_na(name):
+    return 128 if name == "holes128" else 384
+
+
+def stress_blob(name, kind="int8"):
+    """DNNw blob of a stress model: kind int8 | float."""
+    common, only8, onlyf = make_stress_model(name)
+    return blob_bytes(common + (only8 if kind == "int8" else onlyf))
 
 
 NNET_DATA_H = """/* Generated by oracle/gen_model.py in the format of training_tf2/dump_lpcnet.py:303-385 */

@@ -116,6 +116,7 @@ typedef struct {
     float vq_mem[NB_BANDS];      /* LPCNetDecState.vq_mem */
     /* optional trace of the last synthesize call */
     int *trace_exc;              /* if non-NULL: exc index per generated sample */
+    int32_t acc_peak;            /* int8: largest |GRU_A accumulator| (entry value or final sum) since the last reset */
 } OState;
 
 /* ------------------------------------------------------------------ blob ------------------------------------------------------------------ */
@@ -475,21 +476,25 @@ static void run_frame_network(OState *st, const float *features)     /* lpcnet.c
 #define SCALE_1 (1.f / 128.f / 127.f)
 
 /* int8: sparse_sgemv_accum8x4 vec_avx.h:790-858 ; float: vec_avx.h:865-903 */
-static void sparse_gemv(const OModel *m, float *out, const void *wv, int rows, int cols, const int *idx, const float *xin)
+static void sparse_gemv(const OModel *m, float *out, const void *wv, int rows, int cols, const int *idx, const float *xin, int32_t *peak)
 {
     int i, j, r, c;
     if (!m->is_float) {
         const signed char *w = wv; unsigned char x[N_A_MAX];
         for (i = 0; i < cols; i++) x[i] = quant_u8(xin[i]);
         for (i = 0; i < rows; i += 8) {
-            int nb = *idx++; int32_t acc[8];
-            for (r = 0; r < 8; r++) acc[r] = (int32_t)lrintf(out[i + r] * SCALE);
+            int nb = *idx++; int32_t acc[8], acc0[8];
+            for (r = 0; r < 8; r++) acc0[r] = acc[r] = (int32_t)lrintf(out[i + r] * SCALE);
             for (j = 0; j < nb; j++) {
                 int pos = *idx++;
                 for (r = 0; r < 8; r++) for (c = 0; c < 4; c++) acc[r] += (int)x[pos + c] * (int)w[r * 4 + c];
                 w += 32;
             }
             for (r = 0; r < 8; r++) out[i + r] = (float)acc[r] * SCALE_1;
+            if (peak) for (r = 0; r < 8; r++) {
+                if (abs(acc0[r]) > *peak) *peak = abs(acc0[r]);
+                if (abs(acc[r]) > *peak) *peak = abs(acc[r]);
+            }
         }
     } else {
         const float *w = wv;
@@ -522,7 +527,7 @@ static int run_sample_network(OState *st, int last_exc, int last_sig, int pred) 
     bias = m->is_float ? &m->ga_bias[3 * N_A] : &m->ga_subias[3 * N_A];
     for (k = 0; k < 2; k++) for (i = 0; i < N_A; i++) recur[k * N_A + i] = bias[k * N_A + i] + m->ga_diag[k * N_A + i] * state[i] + gin[k * N_A + i];
     for (; k < 3; k++) for (i = 0; i < N_A; i++) recur[k * N_A + i] = bias[k * N_A + i] + m->ga_diag[k * N_A + i] * state[i];
-    sparse_gemv(m, recur, m->ga_w, 3 * N_A, N_A, m->ga_idx, state);
+    sparse_gemv(m, recur, m->ga_w, 3 * N_A, N_A, m->ga_idx, state, &st->acc_peak);
     for (i = 0; i < 2 * N_A; i++) recur[i] = sigmoid_a(m, recur[i]);
     for (i = 0; i < N_A; i++) recur[2 * N_A + i] = recur[2 * N_A + i] * recur[N_A + i] + gin[2 * N_A + i];
     for (i = 0; i < N_A; i++) recur[2 * N_A + i] = tanh_a(m, recur[2 * N_A + i]);
@@ -530,7 +535,7 @@ static int run_sample_network(OState *st, int last_exc, int last_sig, int pred) 
     /* compute_gruB nnet.c:326-372 */
     bias = m->is_float ? m->gb_bias : m->gb_subias;
     for (i = 0; i < 3 * N_B; i++) zrh[i] = bias[i] + st->gru_b_condition[i];
-    sparse_gemv(m, zrh, m->gb_w, 3 * N_B, N_A, m->gb_idx, state);
+    sparse_gemv(m, zrh, m->gb_w, 3 * N_B, N_A, m->gb_idx, state, NULL);
     for (i = 0; i < 3 * N_B; i++) rec_b[i] = bias[3 * N_B + i];
     if (!m->is_float) {                                        /* sgemv_accum8x4 vec_avx.h:690-755 */
         const signed char *w = m->gb_rw; unsigned char x[N_B]; int r, c;
@@ -751,6 +756,10 @@ int oracle_export_state(const OState *st, float *buf)
     memcpy(buf + o, iv, sizeof(iv)); o += 6;
     return o * 4;
 }
+/* int8 models: largest |accumulator| of the GRU_A GEMV seen by this state (the conversion-free rounding of the CUDA kernel is exact
+   below 2^22; model.cu proves a bound from the weights, this measures what synthesis reaches) */
+int oracle_acc_peak(const OState *st) { return st->acc_peak; }
+
 void oracle_synthesize_trace(OState *st, const float *features, short *output, int N, int *exc)
 {
     st->trace_exc = exc; oracle_synthesize(st, features, output, N); st->trace_exc = NULL;

@@ -81,6 +81,7 @@ def oracle_lib():
     L.oracle_reset.argtypes = [c_p]
     L.oracle_synthesize.argtypes = [c_p, c_p, c_p, ctypes.c_int]
     L.oracle_synthesize_trace.argtypes = [c_p, c_p, c_p, ctypes.c_int, c_p]
+    L.oracle_acc_peak.argtypes = [c_p]
     L.oracle_decode.argtypes = [c_p, c_p, c_p]
     L.oracle_decode_packet.argtypes = [c_p, c_p, c_p]
     L.oracle_frame_network.argtypes = [c_p, c_p, c_p, c_p, c_p]
@@ -105,23 +106,38 @@ def oracle_lib():
 
 
 @functools.lru_cache(None)
-def oracle_model(kind="int8", tag=""):
-    """CPU-restatement model for a blob flavour (int8 / float / int8_clamp) of a model variant (tag, gen_model.VARIANTS)."""
+def stress_blob(name, kind="int8"):
+    """Blob (int8 | float) of a stress model, gen_model.make_stress_model; generated in memory."""
+    import gen_model
+    return gen_model.stress_blob(name, kind)
+
+
+def stress_tag(name):
+    """The model variant whose generated header (GRU_A size) a stress model shares: selects the compiled reference build."""
+    import gen_model
+    return {128: "na128", 256: "na256", 384: ""}[gen_model.stress_na(name)]
+
+
+@functools.lru_cache(None)
+def oracle_model(kind="int8", tag="", stress=""):
+    """CPU-restatement model for a blob flavour (int8 / float / int8_clamp) of a model variant (tag, gen_model.VARIANTS) or of
+    a stress model (stress, gen_model.STRESS_NAMES; tag is then its stress_tag)."""
     L = oracle_lib()
-    b = blob(kind, tag)
+    b = stress_blob(stress, kind) if stress else blob(kind, tag)
     gamma, delay, e2e = model_config(tag)
     m = L.oracle_model_create_ex(b, len(b), rcp_table().ctypes.data, gamma, delay, int(e2e), codebooks().ctypes.data)
     assert m, "oracle failed to parse the blob"
     return m
 
 
-def oracle_synth(features, kind="int8", nthreads=8, tag=""):
+def oracle_synth(features, kind="int8", nthreads=8, tag="", stress=""):
     """features [n][T][20] float32 -> pcm [n][T*160] int16 via the CPU restatement."""
     L = oracle_lib()
     f = np.ascontiguousarray(features, dtype=np.float32)
     n, T, stride = f.shape
     pcm = np.zeros((n, T * 160), dtype=np.int16)
-    L.oracle_synthesize_batch(oracle_model(kind, tag), f.ctypes.data, stride, n, T, nthreads, pcm.ctypes.data)
+    m = oracle_model(kind, stress_tag(stress), stress) if stress else oracle_model(kind, tag)
+    L.oracle_synthesize_batch(m, f.ctypes.data, stride, n, T, nthreads, pcm.ctypes.data)
     return pcm
 
 
@@ -174,10 +190,13 @@ def ref_lib(build="A", tag=""):
     return L
 
 
-def ref_synth(features, build="A", tag="", kind=None, nthreads=None):
+def ref_synth(features, build="A", tag="", kind=None, nthreads=None, stress=""):
     """features [n][T][stride] -> pcm [n][T*160] through the compiled reference (fresh lpcnet_create() per stream)."""
+    kind = kind or ("float" if build in ("B", "TB") else "int8")
+    if stress:
+        tag = stress_tag(stress)
     L = ref_lib(build, tag)
-    b = blob(kind or ("float" if build in ("B", "TB") else "int8"), tag)
+    b = stress_blob(stress, kind) if stress else blob(kind, tag)
     f = np.ascontiguousarray(features, dtype=np.float32)
     n, T, stride = f.shape
     pcm = np.zeros((n, T * 160), dtype=np.int16)

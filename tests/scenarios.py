@@ -65,8 +65,10 @@ def run_single(backend, lib, st_new, feats, stream, script):
 
 class RefState:
     """state factory for run_single('ref', ...)"""
-    def __init__(self, build="A", tag="", kind=None):
-        self.L = H.ref_lib(build, tag); self.b = H.blob(kind or ("float" if build == "B" else "int8"), tag)
+    def __init__(self, build="A", tag="", kind=None, stress=""):
+        kind = kind or ("float" if build == "B" else "int8")
+        tag = H.stress_tag(stress) if stress else tag
+        self.L = H.ref_lib(build, tag); self.b = H.stress_blob(stress, kind) if stress else H.blob(kind, tag)
     def __call__(self):
         st = self.L.ref_state_create(self.b, len(self.b)); assert st; return st
     def copy_of(self, st):
@@ -76,8 +78,8 @@ class RefState:
 
 
 class OracleState:
-    def __init__(self, kind="int8", tag=""):
-        self.L = H.oracle_lib(); self.m = H.oracle_model(kind, tag)
+    def __init__(self, kind="int8", tag="", stress=""):
+        self.L = H.oracle_lib(); self.m = H.oracle_model(kind, H.stress_tag(stress), stress) if stress else H.oracle_model(kind, tag)
         self.size = 1 << 16
     def __call__(self):
         return self.L.oracle_state_create(self.m)

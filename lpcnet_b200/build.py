@@ -56,7 +56,7 @@ def needs_build():
 
 
 def build_variant(name, defines):
-    """Tuning aid: build lpcnet_b200/variants/lib_<name>.so with extra -D flags (e.g. LPCNET_NWC=12)."""
+    """Tuning aid: build lpcnet_b200/variants/lib_<name>.so with extra -D flags (e.g. LPCNET_TRACE=1)."""
     vdir = os.path.join(HERE, "variants")
     log = []
     os.makedirs(vdir, exist_ok=True)

@@ -206,13 +206,5 @@ __device__ __forceinline__ uint32_t kiss99_rand(Kiss99 &t)
 }
 
 __device__ __forceinline__ float4 ldg4(const float *p) { return __ldg(reinterpret_cast<const float4 *>(p)); }
-// read-only 16-byte load that does not allocate in L1 (the gathered embedding rows have no reuse there; the small L1 left
-// beside 227 KB of shared memory is kept for the sampler's dual_fc rows)
-__device__ __forceinline__ float4 ldg4_stream(const float *p)
-{
-    float4 v;
-    asm volatile("ld.global.nc.L1::no_allocate.v4.f32 {%0, %1, %2, %3}, [%4];" : "=f"(v.x), "=f"(v.y), "=f"(v.z), "=f"(v.w) : "l"(p));
-    return v;
-}
 
 }  // namespace lpcnet_b200

@@ -33,29 +33,24 @@ constexpr int NA_MAX = 384;
 
 // ---- per-sample kernel geometry (warp-specialised CTA) ----
 constexpr int STREAMS_PER_CTA = 32;          // stream slots of a CTA; the launcher may leave some dead (SampleParams::spc) to spread a small batch over all SMs
-#ifndef LPCNET_NWC
-#define LPCNET_NWC 16
-#endif
-constexpr int NWC = LPCNET_NWC;              // compute warps (12, 16 or 24): each owns NGRP/NWC neuron groups of GRU_A, a (row group, K part) of the
-                                             // GRU_B input GEMV and up to ceil(16/NWC) GRU_B neurons.  24 warps x 2 groups keeps the per-thread
-                                             // working set small (h, S_h, S_z = 48 registers) so that 7 warps per scheduler hide the LDS latency
-#ifndef LPCNET_NWP
-#define LPCNET_NWP 6
-#endif
-constexpr int NWP = LPCNET_NWP;              // producer warps: cooperative gather of the GRU_A input rows.  The gather is latency-bound (L2 hits, ~1k cycles
+constexpr int NWC = 16;                      // compute warps: each owns NGRP/NWC neuron groups of GRU_A; the first NWB also walk a (row group, K part)
+                                             // of the GRU_B input GEMV, the last NFIN finish GRU_B (12 and 24 compute warps measured slower, DESIGN.md 4.1)
+constexpr int NWP = 6;                       // producer warps: cooperative gather of the GRU_A input rows.  The gather is latency-bound (L2 hits, ~1k cycles
                                              // under load), so what matters is loads in flight: NWP warps x (registers/4) LDG.128 each
 constexpr int SAMPLE_THREADS = (NWC + NWP + 2) * 32;   // + 2 sampler warps, one per half (tree sampler, LPC filter, u-law, de-emphasis)
 constexpr int FCW_ROW = 36;                  // dual_fc row: 32 weights (16 per channel) + {bias0, bias1, factor0, factor1}; 144 B stride = 16 mod 128, so the
                                              // per-lane LDS.128 row reads of lanes on different nodes mostly land in different 4-bank groups
 constexpr int FCW_SMEM_NODES = 64;           // at most the tree levels 0..5 (nodes 1..63) live in shared memory, the rest is read from global (L2);
                                              // a model whose block lists need the room keeps fewer (32, 16, 8: model.cu), the count travels in the image
-constexpr int KPARTS = (NWC >= 24) ? 4 : 2;  // K split of the GRU_B input GEMV
+constexpr int KPARTS = 2;                    // K split of the GRU_B input GEMV
 constexpr int NWB = 6 * KPARTS;              // warps used by the GRU_B input GEMV: (row group 0..5) x (K part)
 static_assert(NWB <= NWC, "one (row group, K part) of GRU_B per compute warp");
 constexpr int HALF = 16;                     // the 32 streams of a CTA are stepped as two halves of 16 (= the M of one MMA), half a sample apart:
                                              // while the sampler / gather of one half run, the compute warps work on the other half
 constexpr int NFIN = NB * HALF / 32;         // compute warps that finish GRU_B for a half: lane = (neuron parity, stream in half)
 static_assert(NFIN <= NWC, "GRU_B finishing warps");
+constexpr int FIN0 = NWC - NFIN;             // the finishing warps are the LAST ones, which carry no (or the least) GRU_B GEMV work; the LPT of model.cu
+                                             // adds their finishing cost to exactly these warps
 constexpr int ACCB_ROW = 20;                 // int32 per output row of the GRU_B partial sums (16 streams + 4 pad: the MMA accumulator stores of a warp
                                              // (rows 2t, columns gid) then fall into 32 different banks)
 constexpr int NTILE = 4;                     // ring of gather tiles, filled in the order (half A: r, z, h), (half B: r, z, h), ...
@@ -83,9 +78,7 @@ constexpr uint32_t al128(uint32_t x) { return (x + 127u) & ~127u; }
 constexpr uint32_t SMEM_RESERVED = 1024;     // shared-window address of dynamic shared memory on sm_100 (probed at batch_create, batch_api.cu)
 constexpr uint32_t T_ACCB = 0;               // the tile that held a half's candidate gate is dead once h~ is computed; until the half's next indices are out
                                              // it carries  int32 [KPARTS][48][ACCB_ROW] partial sums of the GRU_B input GEMV  and
-constexpr uint32_t T_ACCB_BYTES = KPARTS * 3 * NB * ACCB_ROW * 4;      //   float [16 neurons][16 streams] GRU_B state for the sampler in the LAST 1 KB of the tile (Geom::t_hbs):
-                                             // that is inside the tile's last row(s), the only rows whose conditioning vector may not be
-                                             // prefetched into the r tile that takes the slot next (the sampler is still reading; Geom::late_row0)
+constexpr uint32_t T_ACCB_BYTES = KPARTS * 3 * NB * ACCB_ROW * 4;      //   float [16 neurons][16 streams] GRU_B state for the sampler in the LAST 1 KB of the tile (Geom::t_hbs)
 
 // float flavour geometry that does not depend on the GRU_A size
 constexpr int F_NWC = 16, F_KPARTS = 2, F_NWB = 6 * F_KPARTS;
@@ -101,7 +94,6 @@ struct Geom {
                              // column 2t hit 32 different banks per half-warp
     uint32_t tile_bytes;     // one gate of one half: float [16 streams][gin_row]
     uint32_t t_hbs;          // offset of the GRU_B state scratch inside a (dead) candidate-gate tile
-    int late_row0;           // first tile row that overlaps it
     // shared-memory map of the int8 per-sample kernel.  Everything whose size does not depend on the model's sparsity pattern
     // sits at a COMPILE-TIME offset (keeps the addresses out of registers); only the four block-sparse arrays are placed at
     // run-time offsets behind them.  [sm_image, sm_image + image_bytes) is copied verbatim from the global "SMEM image" built
@@ -112,7 +104,6 @@ struct Geom {
     uint32_t sm_idx;         // int32 [2 halves][3][16]: last_sig_ulaw, pred_ulaw, last_exc
     uint32_t sm_mbar;        // mbarriers: image | full[NTILE] | empty[NTILE] | idx[2] | x[2] | accb[2]
     uint32_t mb_image, mb_full, mb_empty, mb_idx, mb_x, mb_accb;
-    uint32_t mb_cond;        // [NTILE]: the conditioning rows of a tile have landed (TMA, complete_tx)
     uint32_t sm_image;
     // image, fixed part (offsets relative to sm_image)
     uint32_t im_logit;       // float [256] sampling_logit_table
@@ -175,7 +166,6 @@ constexpr Geom make_geom(int na)
     g.gin_row = (uint32_t)na + 8u;
     g.tile_bytes = HALF * g.gin_row * 4u;
     g.t_hbs = g.tile_bytes - NB * HALF * 4u;
-    g.late_row0 = (int)(g.t_hbs / (g.gin_row * 4u));
     g.sm_xs = 0;
     g.sm_xb = g.sm_xs + 2 * g.xs_bytes;
     g.sm_tiles = g.sm_xb + 2 * 2 * 4 * HALF * 4;
@@ -183,7 +173,8 @@ constexpr Geom make_geom(int na)
     g.sm_mbar = al128(g.sm_idx + 2 * 3 * HALF * 4);
     g.mb_image = g.sm_mbar; g.mb_full = g.sm_mbar + 8; g.mb_empty = g.mb_full + 8 * NTILE; g.mb_idx = g.mb_empty + 8 * NTILE;
     g.mb_x = g.mb_idx + 16; g.mb_accb = g.mb_x + 16;
-    g.mb_cond = g.sm_mbar + 128;
+    // The 8 * NTILE bytes behind the 128-byte mbarrier block are unused.  They stay: moving sm_image would move the RCPPS alignment
+    // padding and so change the dual_fc rows a model gets and which models fit the shared-memory budget at all.
     g.sm_image = g.sm_mbar + 128 + 8 * NTILE;      // (32-byte aligned: enough for the bulk copies and every vector access into the image)
     g.im_logit = 0;
     g.im_u2l = g.im_logit + 256 * 4;
@@ -258,12 +249,11 @@ static_assert(NGRP % NWC == 0, "compute warps must divide the neuron groups");
 constexpr int XS_BYTES = (int)GEO.xs_bytes, GIN_ROW = (int)GEO.gin_row;
 constexpr uint32_t TILE_BYTES = GEO.tile_bytes;
 constexpr uint32_t T_HBS = GEO.t_hbs;
-constexpr int LATE_ROW0 = GEO.late_row0;
 static_assert(T_ACCB + T_ACCB_BYTES <= T_HBS, "GRU_B scratch must fit inside the gather tile it aliases");
 constexpr uint32_t SM_XS = GEO.sm_xs, SM_XB = GEO.sm_xb, SM_TILES = GEO.sm_tiles, SM_IDX = GEO.sm_idx, SM_MBAR = GEO.sm_mbar;
-constexpr uint32_t MB_IMAGE = GEO.mb_image, MB_FULL = GEO.mb_full, MB_EMPTY = GEO.mb_empty, MB_IDX = GEO.mb_idx, MB_X = GEO.mb_x, MB_ACCB = GEO.mb_accb, MB_COND = GEO.mb_cond;
+constexpr uint32_t MB_IMAGE = GEO.mb_image, MB_FULL = GEO.mb_full, MB_EMPTY = GEO.mb_empty, MB_IDX = GEO.mb_idx, MB_X = GEO.mb_x, MB_ACCB = GEO.mb_accb;
 constexpr uint32_t SM_IMAGE = GEO.sm_image;
-static_assert(MB_ACCB + 16 + 8 <= MB_COND && MB_COND + 8 * NTILE <= SM_IMAGE, "mbarrier block (+ the TMEM base word and the opaque 1.0f behind MB_ACCB)");
+static_assert(MB_ACCB + 16 <= SM_MBAR + 120 && SM_MBAR + 128 <= SM_IMAGE, "mbarrier block (+ the TMEM base word and the opaque 1.0f at SM_MBAR + 120 / 124)");
 constexpr uint32_t IM_LOGIT = GEO.im_logit, IM_U2L = GEO.im_u2l, IM_DIRA = GEO.im_dira, IM_GRPA = GEO.im_grpa, IM_DIRB = GEO.im_dirb, IM_PRE_END = GEO.im_pre_end;
 constexpr uint32_t IM_RCP = GEO.im_rcp, IM_FCWN = GEO.im_fcwn, IM_PARA = GEO.im_para, IM_WBREC = GEO.im_wbrec, IM_PARB = GEO.im_parb, IM_FCW = GEO.im_fcw, IM_VAR = GEO.im_var;
 static_assert((SMEM_RESERVED + SM_IMAGE + IM_RCP) % 8192u == 0, "rcp table alignment");
@@ -360,8 +350,8 @@ struct SampleParams {
 // are packed into existing words)
 
 // gru_a_dense_feature output of one frame (the GRU_A conditioning rows).  int8 flavour: gate-major with the row pitch of a gather tile
-// (na + 8 floats), so that the rows of consecutive streams for one gate are one contiguous piece of memory that a single TMA bulk copy
-// drops into a tile (sample_kernel.cu, gather_half_tma); float flavour: the reference's [stream][3*na].
+// (na + 8 floats), so that the rows of consecutive streams for one gate are one contiguous piece of memory laid out like a tile
+// (sample_kernel.cu, gather_half); float flavour: the reference's [stream][3*na].
 inline size_t condA_frame_floats(bool is_float, size_t n, int na) { return is_float ? n * 3 * (size_t)na : 3 * n * (size_t)(na + 8); }
 
 // ---- host-side API of the internal modules ----

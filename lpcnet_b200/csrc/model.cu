@@ -226,13 +226,12 @@ static int build_host_model(DeviceModel *m, HostModel &hm, const unsigned char *
     std::vector<int> load(nwc, 0);
     if (!is_float) {
         // The compute warps do not carry the same load besides GRU_A: warps < 6*KPARTS also walk a (row group, K part) of the dense GRU_B
-        // input GEMV (blocks counted like GRU_A's), the last NFIN warps finish GRU_B (worth about `fin` blocks).  Starting the LPT from these
-        // loads hands the heavier neuron groups to the warps with less GRU_B work (LPCNET_B200_LPT="<GRU_B block weight>,<finish cost>").
-        int wgt = 1, fin = 48;                                   // measured: 18.9 -> 18.6 ms per 1600 samples at 4096 streams (profiles/r02v_lpt.txt)
-        if (const char *e = getenv("LPCNET_B200_LPT")) sscanf(e, "%d,%d", &wgt, &fin);      // (tuning)
+        // input GEMV (blocks counted like GRU_A's), the NFIN warps from FIN0 on finish GRU_B (worth about `fin` blocks).  Starting the LPT from these
+        // loads hands the heavier neuron groups to the warps with less GRU_B work.
+        const int wgt = 1, fin = 48;                             // measured: 18.9 -> 18.6 ms per 1600 samples at 4096 streams (profiles/r02v_lpt.txt)
         for (int w = 0; w < nwc; w++) {
             if (w < nwb) load[w] += wgt * (int)(rowsB[w / kparts].size() / kparts);
-            if (w >= nwc - NFIN) load[w] += fin;
+            if (w >= FIN0) load[w] += fin;
         }
     }
     for (int g : order) {

@@ -47,51 +47,6 @@
 #include "engine.h"
 #include "devmath.cuh"
 
-#ifndef LPCNET_RCP_ARITH
-#define LPCNET_RCP_ARITH 0     // bit mask of the GRU_A gates (1: r, 2: z, 4: candidate) whose activations use the table-free RCPPS of devmath.cuh
-                               // instead of the shared-memory table (exact either way).  The table costs ~3.4 bank-conflicted wavefronts per
-                               // look-up on the LSU pipe, the arithmetic form 8 more issue slots: all three gates arithmetic (7) measured 5 % slower
-#endif
-#ifndef LPCNET_LDTM_X4
-#define LPCNET_LDTM_X4 1       // fetch the operands of two quads with one tcgen05.ld.x4 (one LDTM + one R2UR less per pair of quads)
-#endif
-#ifndef LPCNET_PACK_ACT
-#define LPCNET_PACK_ACT 1      // GRU_A activations: also the mul -> add pieces run two neurons at a time (oadd2, devmath.cuh)
-#endif
-#ifndef LPCNET_COND_TMA
-#define LPCNET_COND_TMA 0      // 1: the conditioning rows of a gather tile come by TMA ahead of the sampled indices (gather_half_tma below): the tile
-                               // fill drops from 3.7 k to 2.7 k cycles, but the same bytes then cross the shared-memory port twice (TMA write + LDS) and
-                               // the step does not get shorter (measured 1 % longer, profiles/r02q_sweep.txt); kept as a build option (bit-exact in the
-                               // golden / oracle / grid-shape tests of the 384-unit model; the 128- and 256-unit builds of it have not been run)
-#endif
-#ifndef LPCNET_FCW_PREFETCH
-#define LPCNET_FCW_PREFETCH 0  // 1: the sampler prefetches the dual_fc rows of the tree levels that are read from global memory into L1 two levels
-                               // ahead (CCTL.PF1); measured neutral (profiles/r02q_sweep.txt), off
-#endif
-#ifndef LPCNET_EXPERIMENT
-#define LPCNET_EXPERIMENT 0    // timing experiments only (wrong output): 1 = sampler delayed by 1000 cycles, 2 = sampler skips the two lowest tree levels
-#endif
-#ifndef LPCNET_GRUB_FIRST
-#define LPCNET_GRUB_FIRST 3    // bit 0 / bit 1: GRU_B of half A / half B runs right after the half's activations, before the other half's first GEMVs
-                               // (the GRU_B state is what the half's sampler waits for: 19.52 -> 19.05 ms per 1600 samples, profiles/r02r_sweep.txt)
-#endif
-#ifndef LPCNET_FIN_FIRST_WARP
-#define LPCNET_FIN_FIRST_WARP (NWC - NFIN)   // the NFIN compute warps that finish GRU_B: the LAST ones, which carry no (or the least) GRU_B GEMV work
-#endif
-#ifndef LPCNET_TREE_PAR
-#define LPCNET_TREE_PAR 0      // 1: sampler evaluates the seven nodes of the first three tree levels side by side (see the sampler loop); bit-exact but
-                               // 3.9 % slower (19.25 vs 18.53 ms, profiles/r02x_sweep.txt): four more dot products per sample and more spilled state in the
-                               // sampler cost more than the two serial rounds they save
-#endif
-#ifndef LPCNET_GATHER_NOALLOC
-#define LPCNET_GATHER_NOALLOC 0
-#endif
-#if LPCNET_GATHER_NOALLOC
-#define GLD ldg4_stream
-#else
-#define GLD ldg4
-#endif
-
 // tuning builds (-DLPCNET_TRACE): clock64 stamps of CTA 0 for samples 200..207 of a launch
 #ifdef LPCNET_TRACE
 #define TRACE(P_, step_, ev_, lane_) do { if (blockIdx.x == 0 && (lane_) == 0 && (step_) >= 200 && (step_) < 208) (P_).trace[((step_) - 200) * 32 + (ev_)] = clock64(); } while (0)
@@ -119,7 +74,6 @@ enum {
     BAR_HB = 3       // (+ half) finishing warps arrive, sampler waits: GRU_B state of the half's sample is in hBs
 };
 constexpr int CNT_C = NWC * 32, CNT_HB = NFIN * 32 + 32;
-constexpr int FIN0 = LPCNET_FIN_FIRST_WARP;
 __device__ __forceinline__ void bar_arrive(int id, int count) { asm volatile("bar.arrive %0, %1;" ::"r"(id), "r"(count) : "memory"); }
 
 __device__ __forceinline__ void bar_sync(int id, int count) { asm volatile("bar.sync %0, %1;" ::"r"(id), "r"(count) : "memory"); }
@@ -224,11 +178,7 @@ __device__ __forceinline__ void tmem_ld2(uint32_t &w, uint32_t &m, uint32_t tadd
 // the {weights word, meta} pairs of two consecutive quads with one instruction (four columns)
 __device__ __forceinline__ void tmem_ld22(uint32_t &w0, uint32_t &m0, uint32_t &w1, uint32_t &m1, uint32_t taddr)
 {
-#if LPCNET_LDTM_X4
     asm volatile("tcgen05.ld.sync.aligned.32x32b.x4.b32 {%0, %1, %2, %3}, [%4];" : "=r"(w0), "=r"(m0), "=r"(w1), "=r"(m1) : "r"(taddr));
-#else
-    tmem_ld2(w0, m0, taddr); tmem_ld2(w1, m1, taddr + 2);
-#endif
 }
 // four consecutive columns <-> four floats (the fp32 GRU_A state of a lane parks in tensor memory between its activations, see below)
 __device__ __forceinline__ void tmem_ld4f(float (&v)[4], uint32_t taddr)
@@ -340,7 +290,7 @@ __device__ __forceinline__ void gather_half(float *__restrict__ G, const float *
         constexpr int NCH = NA / 128;
         float4 a[NCH], b[NCH], d[NCH], e[NCH];
 #pragma unroll
-        for (int j = 0; j < NCH; j++) { a[j] = GLD(c + 128 * j); b[j] = GLD(e0 + 128 * j); d[j] = GLD(e1 + 128 * j); e[j] = GLD(e2 + 128 * j); }
+        for (int j = 0; j < NCH; j++) { a[j] = ldg4(c + 128 * j); b[j] = ldg4(e0 + 128 * j); d[j] = ldg4(e1 + 128 * j); e[j] = ldg4(e2 + 128 * j); }
         float *g = G + si * GIN_ROW + lane * 4;
 #pragma unroll
         for (int j = 0; j < NCH; j++) {
@@ -350,76 +300,6 @@ __device__ __forceinline__ void gather_half(float *__restrict__ G, const float *
             r.z = __fadd_rn(__fadd_rn(__fadd_rn(a[j].z, b[j].z), d[j].z), e[j].z);
             r.w = __fadd_rn(__fadd_rn(__fadd_rn(a[j].w, b[j].w), d[j].w), e[j].w);
             *reinterpret_cast<float4 *>(g + 128 * j) = r;
-        }
-    }
-}
-
-// The same tile with the conditioning row prefetched.  Of the four rows that make a tile row only three depend on the indices the
-// sampler has just produced; the conditioning row is known a whole frame ahead.  Producer 0 therefore starts one TMA bulk copy per
-// live tile row (NA*4 bytes, straight into the row's place in the tile) for all three tiles of a half-step BEFORE it waits for the
-// indices (kernel body), and the gather proper adds the three embedding rows in place:
-//   G[si][k] = ((G[si][k] + E_sig[a][k]) + E_pred[b][k]) + E_exc[c][k]
-// Three dependent loads per element instead of four: the 12 LDG.128 a lane keeps in flight cover FOUR 128-column row pieces instead of
-// three, and a tile is two latency-bound load batches per producer instead of three (the tile fill is on the serial chain of a
-// sample: indices -> tiles -> activations -> GRU_B -> sampler -> indices).  Work split: rows 0..FULL_ROWS-1 are dealt whole, row
-// p + NWP*b to producer p in batch b; the pieces of the remaining rows go round the producers, one per batch.
-// Rows >= late0 (only for the r tile, which takes the slot the half's GRU_B state scratch lives in: engine.h, Geom::late_row0) could
-// not be prefetched (the sampler may still be reading the scratch): their conditioning piece is loaded here like the others.
-constexpr int FULL_ROWS = (HALF / NWP) * NWP, GATHER_BATCHES = HALF / NWP;
-static_assert((HALF - FULL_ROWS) * (NA / 128) <= GATHER_BATCHES * NWP, "one piece of the shared rows per producer and batch");
-template <bool ONE>
-__device__ __forceinline__ void gather_half_tma(float *__restrict__ G, const float *__restrict__ cond_f, int n, int cta_s0, int hh, int spc, int nl, int late0,
-                                                const float *__restrict__ emb_sig, const float *__restrict__ emb_pred,
-                                                const float *__restrict__ emb_exc, const int *__restrict__ idx_h,
-                                                int gate, int p, int lane)
-{
-    constexpr int NCH = NA / 128;
-    const int col = gate * NA + lane * 4;
-#pragma unroll 1
-    for (int b = 0; b < GATHER_BATCHES; b++) {
-        const int r = p + NWP * b;                               // whole row
-        const int c = p + NWP * b, rs = FULL_ROWS + c / NCH, cj = c % NCH;   // piece cj of shared row rs
-        const bool hasr = r < nl, hass = c < (HALF - FULL_ROWS) * NCH && rs < nl, lates = hass && rs >= late0;
-        float4 B[NCH], D[NCH], E[NCH], sb, sd, se, sc;
-        if (hasr) {
-            const float *e0 = emb_sig + idx_h[r] * (3 * NA) + col;
-            const float *e1 = emb_pred + idx_h[HALF + r] * (3 * NA) + col;
-            const float *e2 = emb_exc + idx_h[2 * HALF + r] * (3 * NA) + col;
-#pragma unroll
-            for (int j = 0; j < NCH; j++) { B[j] = GLD(e0 + 128 * j); D[j] = GLD(e1 + 128 * j); E[j] = GLD(e2 + 128 * j); }
-        }
-        if (hass) {
-            sb = GLD(emb_sig + idx_h[rs] * (3 * NA) + col + 128 * cj);
-            sd = GLD(emb_pred + idx_h[HALF + rs] * (3 * NA) + col + 128 * cj);
-            se = GLD(emb_exc + idx_h[2 * HALF + rs] * (3 * NA) + col + 128 * cj);
-            if (lates) {
-                bool live;
-                const int sg = slot_stream<ONE>(cta_s0, hh, rs, spc, n, live);
-                sc = GLD(cond_row(cond_f, n, gate, sg) + lane * 4 + 128 * cj);
-            }
-        }
-        if (hasr) {
-            float *g = G + r * GIN_ROW + lane * 4;
-#pragma unroll
-            for (int j = 0; j < NCH; j++) {
-                const float4 a = *reinterpret_cast<const float4 *>(g + 128 * j);
-                float4 o;
-                o.x = __fadd_rn(__fadd_rn(__fadd_rn(a.x, B[j].x), D[j].x), E[j].x);
-                o.y = __fadd_rn(__fadd_rn(__fadd_rn(a.y, B[j].y), D[j].y), E[j].y);
-                o.z = __fadd_rn(__fadd_rn(__fadd_rn(a.z, B[j].z), D[j].z), E[j].z);
-                o.w = __fadd_rn(__fadd_rn(__fadd_rn(a.w, B[j].w), D[j].w), E[j].w);
-                *reinterpret_cast<float4 *>(g + 128 * j) = o;
-            }
-        }
-        if (hass) {
-            float *g = G + rs * GIN_ROW + lane * 4 + 128 * cj;
-            if (!lates) sc = *reinterpret_cast<const float4 *>(g);
-            float4 o;
-            o.x = __fadd_rn(__fadd_rn(__fadd_rn(sc.x, sb.x), sd.x), se.x);
-            o.y = __fadd_rn(__fadd_rn(__fadd_rn(sc.y, sb.y), sd.y), se.y);
-            o.z = __fadd_rn(__fadd_rn(__fadd_rn(sc.z, sb.z), sd.z), se.z);
-            o.w = __fadd_rn(__fadd_rn(__fadd_rn(sc.w, sb.w), sd.w), se.w);
-            *reinterpret_cast<float4 *>(g) = o;
         }
     }
 }
@@ -446,9 +326,9 @@ struct ComputeCtx {
 
 // One GRU_A + GRU_B step of half H (16 streams).  k0 = index of the half-step's first tile fill (gate r; z and h follow).
 // A half-step of the compute warps is three pieces:  gemv_rh<H>  |  activations<H> (ends by ARRIVING on MB_X[H])  |  grub<H> (WAITS on MB_X[H]).
-// grub<H> used to run only after the other half's gemv_rh, so that no CTA-wide barrier was waited for right after it was armed; but the
-// GRU_B state is what the half's sampler waits for, i.e. it is on the serial chain of a sample, while a warp that waits at the barrier only
-// gives its issue slots to the others: LPCNET_GRUB_FIRST (default) runs it right behind the activations (-2.9 % per step).
+// grub<H> runs right behind the activations, before the other half's gemv_rh, although it then waits on a CTA-wide barrier right after
+// it was armed: the GRU_B state is what the half's sampler waits for, i.e. it is on the serial chain of a sample, while a warp that waits
+// at the barrier only gives its issue slots to the others (-2.9 % per step against the other order, profiles/r02r_sweep.txt).
 
 // GEMVs of the candidate and reset gates of half H (need only the previous state)
 template <int H>
@@ -479,23 +359,8 @@ __device__ __forceinline__ void activations(const ComputeCtx &C, int (&Sh)[GPW][
 #pragma unroll
     for (int sl = 0; sl < GPW; sl++) tmem_ld4f(h[sl], C.tmH + (H * GPW + sl) * 4);
     uint8_t *smem = C.smem;
-    const int gid = C.gid, t = C.t, lane = C.lane, warp = C.warp;
-    // per-gate choice of the RCPPS implementation (LPCNET_RCP_ARITH mask)
-#if LPCNET_RCP_ARITH & 1
-    const RcpArith rcp_r = RcpArith();
-#else
-    const RcpShared rcp_r = C.rcp;
-#endif
-#if LPCNET_RCP_ARITH & 2
-    const RcpArith rcp_z = RcpArith();
-#else
-    const RcpShared rcp_z = C.rcp;
-#endif
-#if LPCNET_RCP_ARITH & 4
-    const RcpArith rcp_h = RcpArith();
-#else
-    const RcpShared rcp_h = C.rcp;
-#endif
+    const int gid = C.gid, lane = C.lane;
+    const RcpShared rcp = C.rcp;
     const int nxt = cur ^ 1;
     const uint32_t xs_cur = C.xs0 + cur * XS_BYTES, lc = C.gid8 | (H << 6);
     uint8_t *xs_nxt = smem + SM_XS + nxt * XS_BYTES;
@@ -505,7 +370,6 @@ __device__ __forceinline__ void activations(const ComputeCtx &C, int (&Sh)[GPW][
     uint8_t *tile_hb = smem + SM_TILES + (kh & 3) * TILE_BYTES;
     const float *tile_h = reinterpret_cast<const float *>(tile_hb) + gid * GIN_ROW;
     const uint32_t mb_full = smem_u32(smem + MB_FULL), mb_empty = smem_u32(smem + MB_EMPTY);
-    (void)t; (void)warp; (void)rcp_r; (void)rcp_z; (void)rcp_h; (void)nxt; (void)xs_cur; (void)lc; (void)xs_nxt; (void)tile_r; (void)tile_z; (void)tile_h; (void)mb_full; (void)mb_empty; (void)lane;
     // ---- reset gate r (nnet.c:431-435) with the gathered input term; keep rec_h * r (nnet.c:436-440) ----
     mbar_wait(mb_full + 8 * (kr & 3), (kr >> 2) & 1);
 #pragma unroll
@@ -522,7 +386,6 @@ __device__ __forceinline__ void activations(const ComputeCtx &C, int (&Sh)[GPW][
             const float gin[2] = {gv.x, gv.y};
             if constexpr (FAST) {
                 int a[2], ah[2];
-#if LPCNET_PACK_ACT
                 {   // both neurons of the lane at a time; every mul -> add of the reference goes through oadd2
                     const f32x2 hv2 = pk2(h[sl][2 * jj], h[sl][2 * jj + 1]), ONE = C.one2;
                     float a0, a1, b0, b1;
@@ -531,36 +394,21 @@ __device__ __forceinline__ void activations(const ComputeCtx &C, int (&Sh)[GPW][
                     a[0] = __float_as_int(a0) + Sg[sl][2 * jj]; a[1] = __float_as_int(a1) + Sg[sl][2 * jj + 1];
                     ah[0] = __float_as_int(b0) + Sh[sl][2 * jj]; ah[1] = __float_as_int(b1) + Sh[sl][2 * jj + 1];
                 }
-#else
-                // mul -> add pieces scalar, the rest two neurons at a time (devmath.cuh)
-#pragma unroll
-                for (int i = 0; i < 2; i++) {
-                    const float hv = h[sl][2 * jj + i];
-                    a[i] = acc_init_t<true>(__fadd_rn(__fadd_rn(bri[i], __fmul_rn(dri[i], hv)), gin[i])) + Sg[sl][2 * jj + i];
-                    ah[i] = acc_init_t<true>(__fadd_rn(bhi[i], __fmul_rn(dhi[i], hv))) + Sh[sl][2 * jj + i];
-                }
-#endif
                 f32x2 num, den;
                 rational2(acc_finish2(a[0], a[1]), LPCNET_SIGMOID_COEF, num, den);
                 float n0, n1, d0, d1, rh0, rh1;
                 upk2(num, n0, n1); upk2(den, d0, d1);
-                const float r0 = fmaxf(0.f, fminf(1.f, __fmaf_rn(n0, rcp_emul(d0, rcp_r), 0.5f)));
-                const float r1 = fmaxf(0.f, fminf(1.f, __fmaf_rn(n1, rcp_emul(d1, rcp_r), 0.5f)));
-#if LPCNET_PACK_ACT
+                const float r0 = fmaxf(0.f, fminf(1.f, __fmaf_rn(n0, rcp_emul(d0, rcp), 0.5f)));
+                const float r1 = fmaxf(0.f, fminf(1.f, __fmaf_rn(n1, rcp_emul(d1, rcp), 0.5f)));
                 upk2(mul2(acc_finish2(ah[0], ah[1]), pk2(r0, r1)), rh0, rh1);
                 Sh[sl][2 * jj] = __float_as_int(rh0);
                 Sh[sl][2 * jj + 1] = __float_as_int(rh1);
-#else
-                upk2(acc_finish2(ah[0], ah[1]), rh0, rh1);
-                Sh[sl][2 * jj] = __float_as_int(__fmul_rn(rh0, r0));
-                Sh[sl][2 * jj + 1] = __float_as_int(__fmul_rn(rh1, r1));
-#endif
             } else {
 #pragma unroll
                 for (int i = 0; i < 2; i++) {
                     const float hv = h[sl][2 * jj + i];
                     const int acc = acc_init_t<FAST>(__fadd_rn(__fadd_rn(bri[i], __fmul_rn(dri[i], hv)), gin[i])) + Sg[sl][2 * jj + i];
-                    const float r = sigmoid_approx(acc_finish_t<FAST>(acc), rcp_r);
+                    const float r = sigmoid_approx(acc_finish_t<FAST>(acc), rcp);
                     const int acch = acc_init_t<FAST>(__fadd_rn(bhi[i], __fmul_rn(dhi[i], hv))) + Sh[sl][2 * jj + i];
                     Sh[sl][2 * jj + i] = __float_as_int(__fmul_rn(acc_finish_t<FAST>(acch), r));
                 }
@@ -592,29 +440,23 @@ __device__ __forceinline__ void activations(const ComputeCtx &C, int (&Sh)[GPW][
             const float gin[2] = {gv.x, gv.y};
             if constexpr (FAST) {
                 int a[2];
-#if LPCNET_PACK_ACT
                 {
                     const f32x2 ONE = C.one2;
                     float a0, a1;
                     upk2(oadd2(mul2(add2(oadd2(mul2(pk2(dz.x, dz.y), pk2(h[sl][2 * jj], h[sl][2 * jj + 1])), ONE, pk2(bz.x, bz.y)), pk2(gv.x, gv.y)), k2(LPCNET_SCALE)), ONE, k2(LPCNET_CVT_MAGIC)), a0, a1);
                     a[0] = __float_as_int(a0) + Sg[sl][2 * jj]; a[1] = __float_as_int(a1) + Sg[sl][2 * jj + 1];
                 }
-#else
-#pragma unroll
-                for (int i = 0; i < 2; i++)
-                    a[i] = acc_init_t<true>(__fadd_rn(__fadd_rn(bzi[i], __fmul_rn(dzi[i], h[sl][2 * jj + i])), gin[i])) + Sg[sl][2 * jj + i];
-#endif
                 f32x2 num, den;
                 rational2(acc_finish2(a[0], a[1]), LPCNET_SIGMOID_COEF, num, den);
                 float n0, n1, d0, d1;
                 upk2(num, n0, n1); upk2(den, d0, d1);
-                Sg[sl][2 * jj] = __float_as_int(fmaxf(0.f, fminf(1.f, __fmaf_rn(n0, rcp_emul(d0, rcp_z), 0.5f))));
-                Sg[sl][2 * jj + 1] = __float_as_int(fmaxf(0.f, fminf(1.f, __fmaf_rn(n1, rcp_emul(d1, rcp_z), 0.5f))));
+                Sg[sl][2 * jj] = __float_as_int(fmaxf(0.f, fminf(1.f, __fmaf_rn(n0, rcp_emul(d0, rcp), 0.5f))));
+                Sg[sl][2 * jj + 1] = __float_as_int(fmaxf(0.f, fminf(1.f, __fmaf_rn(n1, rcp_emul(d1, rcp), 0.5f))));
             } else {
 #pragma unroll
                 for (int i = 0; i < 2; i++) {
                     const int acc = acc_init_t<FAST>(__fadd_rn(__fadd_rn(bzi[i], __fmul_rn(dzi[i], h[sl][2 * jj + i])), gin[i])) + Sg[sl][2 * jj + i];
-                    Sg[sl][2 * jj + i] = __float_as_int(sigmoid_approx(acc_finish_t<FAST>(acc), rcp_z));
+                    Sg[sl][2 * jj + i] = __float_as_int(sigmoid_approx(acc_finish_t<FAST>(acc), rcp));
                 }
             }
         }
@@ -634,23 +476,14 @@ __device__ __forceinline__ void activations(const ComputeCtx &C, int (&Sh)[GPW][
                 rational2(add2(pk2(__int_as_float(Sh[sl][2 * jj]), __int_as_float(Sh[sl][2 * jj + 1])), pk2(gin[0], gin[1])), LPCNET_TANH_COEF, num, den);
                 float d0, d1, t0, t1;
                 upk2(den, d0, d1);
-                upk2(mul2(num, pk2(rcp_emul(d0, rcp_h), rcp_emul(d1, rcp_h))), t0, t1);
+                upk2(mul2(num, pk2(rcp_emul(d0, rcp), rcp_emul(d1, rcp))), t0, t1);
                 const float hh[2] = {fmaxf(-1.f, fminf(1.f, t0)), fmaxf(-1.f, fminf(1.f, t1))};
                 float hn[2];
-#if LPCNET_PACK_ACT
                 {
                     const f32x2 z2 = pk2(__int_as_float(Sg[sl][2 * jj]), __int_as_float(Sg[sl][2 * jj + 1]));
                     upk2(oadd2(mul2(z2, pk2(h[sl][2 * jj], h[sl][2 * jj + 1])), C.one2, mul2(one_minus2(z2), pk2(hh[0], hh[1]))), hn[0], hn[1]);
                     h[sl][2 * jj] = hn[0]; h[sl][2 * jj + 1] = hn[1];
                 }
-#else
-#pragma unroll
-                for (int i = 0; i < 2; i++) {
-                    const float z = __int_as_float(Sg[sl][2 * jj + i]);
-                    hn[i] = __fadd_rn(__fmul_rn(z, h[sl][2 * jj + i]), __fmul_rn(__fsub_rn(1.f, z), hh[i]));
-                    h[sl][2 * jj + i] = hn[i];
-                }
-#endif
                 // quantised bytes in the low bytes of the biased patterns: fma -> add, safe to pack
                 float q0, q1;
                 upk2(add2(fma2(pk2(hn[0], hn[1]), k2(127.f), k2(127.f)), k2(LPCNET_CVT_MAGIC)), q0, q1);
@@ -658,7 +491,7 @@ __device__ __forceinline__ void activations(const ComputeCtx &C, int (&Sh)[GPW][
             } else {
 #pragma unroll
                 for (int i = 0; i < 2; i++) {
-                    const float hh = tanh_approx(__fadd_rn(__int_as_float(Sh[sl][2 * jj + i]), gin[i]), rcp_h);
+                    const float hh = tanh_approx(__fadd_rn(__int_as_float(Sh[sl][2 * jj + i]), gin[i]), rcp);
                     const float z = __int_as_float(Sg[sl][2 * jj + i]);
                     const float hn = __fadd_rn(__fmul_rn(z, h[sl][2 * jj + i]), __fmul_rn(__fsub_rn(1.f, z), hh));
                     h[sl][2 * jj + i] = hn;
@@ -681,15 +514,10 @@ __device__ __forceinline__ void grub(const ComputeCtx &C, const SampleParams &P,
     const int gid = C.gid, t = C.t, lane = C.lane, warp = C.warp;
     const RcpShared rcp = C.rcp;
     const int nxt = cur ^ 1;
-    const uint32_t xs_cur = C.xs0 + cur * XS_BYTES, lc = C.gid8 | (H << 6);
-    uint8_t *xs_nxt = smem + SM_XS + nxt * XS_BYTES;
-    const uint32_t kr = k0, kz = k0 + 1, kh = k0 + 2;
-    const float *tile_r = reinterpret_cast<const float *>(smem + SM_TILES + (kr & 3) * TILE_BYTES) + gid * GIN_ROW;
-    const float *tile_z = reinterpret_cast<const float *>(smem + SM_TILES + (kz & 3) * TILE_BYTES) + gid * GIN_ROW;
+    const uint32_t lc = C.gid8 | (H << 6);
+    const uint32_t kh = k0 + 2;
     uint8_t *tile_hb = smem + SM_TILES + (kh & 3) * TILE_BYTES;
-    const float *tile_h = reinterpret_cast<const float *>(tile_hb) + gid * GIN_ROW;
-    const uint32_t mb_full = smem_u32(smem + MB_FULL), mb_empty = smem_u32(smem + MB_EMPTY);
-    (void)t; (void)warp; (void)rcp; (void)nxt; (void)xs_cur; (void)lc; (void)xs_nxt; (void)tile_r; (void)tile_z; (void)tile_h; (void)mb_full; (void)mb_empty; (void)lane;
+    const uint32_t mb_empty = smem_u32(smem + MB_EMPTY);
     mbar_wait(smem_u32(smem + MB_X) + 8 * H, par);               // new quantised GRU_A state complete; candidate-gate tile dead: GRU_B scratch may use it
     TRACEC(P, trstep, 27, warp == 0 ? lane : 1);
     // ---------------- GRU_B input GEMV (48 x 384 int8, dense): warp = (row group, K part) ----------------
@@ -764,7 +592,6 @@ __global__ void __launch_bounds__(SAMPLE_THREADS, 1) lpcnet_sample_kernel(const 
     if (threadIdx.x == 0) {
         mbar_init(bar, 1);
         for (int b = 0; b < NTILE; b++) { mbar_init(smem_u32(smem + MB_FULL) + 8 * b, NWP * ARRIVALS_PER_WARP); mbar_init(smem_u32(smem + MB_EMPTY) + 8 * b, NWC * ARRIVALS_PER_WARP); }
-        for (int b = 0; b < NTILE; b++) mbar_init(smem_u32(smem + MB_COND) + 8 * b, 1);
         for (int hh = 0; hh < 2; hh++) { mbar_init(smem_u32(smem + MB_IDX) + 8 * hh, ARRIVALS_PER_WARP); mbar_init(smem_u32(smem + MB_X) + 8 * hh, NWC * ARRIVALS_PER_WARP); mbar_init(smem_u32(smem + MB_ACCB) + 8 * hh, NWB * ARRIVALS_PER_WARP); }
         asm volatile("fence.mbarrier_init.release.cluster;" ::: "memory");
     }
@@ -882,29 +709,17 @@ __global__ void __launch_bounds__(SAMPLE_THREADS, 1) lpcnet_sample_kernel(const 
                 int Sh[GPW][4], Sg[GPW][4];                              // candidate-gate sums (later rec_h * r) / r-gate, then z-gate sums (later z)
                 const int tl = warp == 0 ? lane : 1; (void)tl;    // (lane selector of the TRACE stamps)
                 TRACEC(P, step, 0, tl); TRACEW(P, step, 0);
-#if LPCNET_GRUB_FIRST & 2
                 if (step > 0) grub<1, FAST>(C, P, hb[1], k - 3, (step - 1) & 1, f_prev, s_fin[1], (step - 1) & 1);
                 TRACEC(P, step, 1, tl); TRACEW(P, step, 1);
                 gemv_rh<0>(C, Sh, Sg, step & 1);
-#else
-                gemv_rh<0>(C, Sh, Sg, step & 1);
-                TRACEC(P, step, 1, tl); TRACEW(P, step, 1);
-                if (step > 0) grub<1, FAST>(C, P, hb[1], k - 3, (step - 1) & 1, f_prev, s_fin[1], (step - 1) & 1);
-#endif
                 TRACEC(P, step, 2, tl); TRACEW(P, step, 2);       // = HB of half B (previous sample) signalled
                 mbar_wait(smem_u32(smem + MB_FULL) + 8 * (k & 3), (k >> 2) & 1);
                 TRACEC(P, step, 3, tl); TRACEW(P, step, 3);       // r tile of half A present
                 activations<0, FAST>(C, Sh, Sg, k, step & 1);
                 TRACEC(P, step, 4, tl); TRACEW(P, step, 4);
-#if LPCNET_GRUB_FIRST & 1
                 grub<0, FAST>(C, P, hb[0], k, step & 1, f, s_fin[0], step & 1, step);
                 TRACEC(P, step, 5, tl); TRACEW(P, step, 5);
                 gemv_rh<1>(C, Sh, Sg, step & 1);
-#else
-                gemv_rh<1>(C, Sh, Sg, step & 1);
-                TRACEC(P, step, 5, tl); TRACEW(P, step, 5);
-                grub<0, FAST>(C, P, hb[0], k, step & 1, f, s_fin[0], step & 1, step);
-#endif
                 TRACEC(P, step, 6, tl); TRACEW(P, step, 6);       // = HB of half A signalled
                 mbar_wait(smem_u32(smem + MB_FULL) + 8 * ((k + 3) & 3), ((k + 3) >> 2) & 1);
                 TRACEC(P, step, 7, tl); TRACEW(P, step, 7);       // r tile of half B present
@@ -946,55 +761,19 @@ __global__ void __launch_bounds__(SAMPLE_THREADS, 1) lpcnet_sample_kernel(const 
         const int p = warp - NWC;
         const uint32_t mb_full = smem_u32(smem + MB_FULL), mb_empty = smem_u32(smem + MB_EMPTY), mb_idx = smem_u32(smem + MB_IDX);
         uint32_t k = 0, it = 0;
-#if LPCNET_COND_TMA
-        const uint32_t mb_cond = smem_u32(smem + MB_COND);
-        int nlive[2] = {0, 0};                                           // live tile rows of the halves (the live slots of a half are its first rows)
-        for (int hh = 0; hh < 2; hh++)
-            for (int si = 0; si < HALF; si++) { bool live; slot_stream<ONE>(cta_s0, hh, si, spc, n, live); nlive[hh] += live ? 1 : 0; }
-#endif
         for (int f = 0; f < P.nframes; f++) {
             const float *condA_f = P.condA + (size_t)f * n * (3 * GIN_ROW);
             for (int t_ = 0; t_ < spf; t_++, it++)
 #pragma unroll 1
                 for (int hh = 0; hh < (one ? 1 : 2); hh++) {
-#if LPCNET_COND_TMA
-                    const int nl = nlive[hh];
-                    if (p == 0) {
-                        // conditioning rows of the half-step's three tiles, ahead of the indices (gather_half_tma).  A slot is written only
-                        // after every compute warp has released its previous contents; the r tile takes the slot whose last rows hold the
-                        // half's GRU_B state scratch, which the sampler reads until it publishes the indices: those rows are left out here.
-#pragma unroll 1
-                        for (int gi = 0; gi < 3; gi++) {
-                            const uint32_t kk = k + gi;
-                            const int gate = gi == 0 ? 1 : (gi == 1 ? 0 : 2), rows = gi == 0 ? min(nl, LATE_ROW0) : nl;
-                            mbar_wait(mb_empty + 8 * (kk & 3), ((kk >> 2) & 1) ^ 1);
-                            if (lane == 0) {
-                                asm volatile("fence.proxy.async.shared::cta;" ::: "memory");      // generic accesses of the old contents before the async-proxy writes
-                                mbar_expect_tx(mb_cond + 8 * (kk & 3), (uint32_t)rows * (GIN_ROW * 4));
-                                if (rows > 0) {                                              // the rows of a half are consecutive streams: ONE bulk copy, pitch = tile pitch
-                                    bool live;
-                                    const int sg0 = slot_stream<ONE>(cta_s0, hh, 0, spc, n, live);
-                                    bulk_g2s(smem_u32(smem + SM_TILES + (kk & 3) * TILE_BYTES), cond_row(condA_f, n, gate, sg0), (uint32_t)rows * (GIN_ROW * 4), mb_cond + 8 * (kk & 3));
-                                }
-                            }
-                            __syncwarp();
-                        }
-                    }
-#endif
                     mbar_wait(mb_idx + 8 * hh, it & 1);                  // indices of this sample of the half are in idx_s
                     TRACE(P, (int)it, 10 + 4 * hh, p == 0 ? lane : 1);
 #pragma unroll 1
                     for (int gi = 0; gi < 3; gi++, k++) {
                         const int gate = gi == 0 ? 1 : (gi == 1 ? 0 : 2);    // fill order r, z, h
-#if LPCNET_COND_TMA
-                        mbar_wait(mb_cond + 8 * (k & 3), (k >> 2) & 1);      // conditioning rows landed (issued after the slot was released)
-                        gather_half_tma<ONE>(reinterpret_cast<float *>(smem + SM_TILES + (k & 3) * TILE_BYTES), condA_f, n, cta_s0, hh, spc, nl, gi == 0 ? LATE_ROW0 : HALF,
-                                    P.emb_sig, P.emb_pred, P.emb_exc, idx_s + hh * 3 * HALF, gate, p, lane);
-#else
                         mbar_wait(mb_empty + 8 * (k & 3), ((k >> 2) & 1) ^ 1);  // previous contents of the tile consumed
                         gather_half<ONE>(reinterpret_cast<float *>(smem + SM_TILES + (k & 3) * TILE_BYTES), condA_f, n, cta_s0, hh, spc,
                                     P.emb_sig, P.emb_pred, P.emb_exc, idx_s + hh * 3 * HALF, gate, p, lane);
-#endif
                         warp_arrive(mb_full + 8 * (k & 3), lane);
                         TRACE(P, (int)it, 11 + 4 * hh + gi, p == 0 ? lane : 1);
                     }
@@ -1069,36 +848,8 @@ __global__ void __launch_bounds__(SAMPLE_THREADS, 1) lpcnet_sample_kernel(const 
 #pragma unroll
                 for (int j = 0; j < NB; j++) hbv[j] = hBs[j * HALF + si];
                 int val = 0;
-#if LPCNET_EXPERIMENT == 1
-                { const long long t0 = clock64(); while (clock64() - t0 < 1000) { } }      // (timing experiment: a slower sampler)
-#endif
-#if LPCNET_TREE_PAR
-                // The nodes of the first three tree levels (1..7, rows always in shared memory) do not depend on any decision: all seven are
-                // evaluated side by side (seven independent 16-term chains interleave in the pipeline) and the three decisions are then just
-                // compares, instead of three strictly serial load -> chain -> tanh -> shuffle -> compare rounds on the sample's critical path.
-                {
-                    float totn[8];
 #pragma unroll
-                    for (int nd = 1; nd < 8; nd++) {
-                        const float *wr = fcw + nd * FCW_ROW;
-                        const float4 a0 = *reinterpret_cast<const float4 *>(wr), a1 = *reinterpret_cast<const float4 *>(wr + 4);
-                        const float4 a2 = *reinterpret_cast<const float4 *>(wr + 8), a3 = *reinterpret_cast<const float4 *>(wr + 12);
-                        const float w16[16] = {a0.x, a0.y, a0.z, a0.w, a1.x, a1.y, a1.z, a1.w, a2.x, a2.y, a2.z, a2.w, a3.x, a3.y, a3.z, a3.w};
-                        float sum = wr[2 * NB - ch * NB + ch];
-                        const float fac = wr[2 * NB - ch * NB + 2 + ch];
-#pragma unroll
-                        for (int j = 0; j < NB; j++) sum = __fadd_rn(sum, __fmul_rn(w16[j], hbv[j]));
-                        const float mine = __fmul_rn(fac, tanh_approx(sum, rcp));
-                        totn[nd] = __fadd_rn(mine, __shfl_xor_sync(0xffffffffu, mine, 16));
-                    }
-                    val = thr[0] < totn[1] ? 1 : 0;
-                    val = (val << 1) | (thr[1] < (val ? totn[3] : totn[2]) ? 1 : 0);
-                    const float t3 = (val & 2) ? ((val & 1) ? totn[7] : totn[6]) : ((val & 1) ? totn[5] : totn[4]);
-                    val = (val << 1) | (thr[2] < t3 ? 1 : 0);
-                }
-#endif
-#pragma unroll
-                for (int b = (LPCNET_TREE_PAR ? 3 : 0); b < (LPCNET_EXPERIMENT == 2 ? 6 : 8); b++) {                            // sample_mdense, nnet.c:186-211
+                for (int b = 0; b < 8; b++) {                            // sample_mdense, nnet.c:186-211
                     const int i = (1 << b) | val;
                     // this lane's channel: a sequential 16-term chain
                     float w16[16], sum, fac;
@@ -1122,21 +873,6 @@ __global__ void __launch_bounds__(SAMPLE_THREADS, 1) lpcnet_sample_kernel(const 
                     const float other = __shfl_xor_sync(0xffffffffu, mine, 16);
                     const float tot = __fadd_rn(mine, other);            // channel 0 + channel 1 (commutative: both lanes get the same bits)
                     val = (val << 1) | (thr[b] < tot ? 1 : 0);
-#if LPCNET_FCW_PREFETCH
-                    // The node of level b+2 is one of two adjacent rows (288 bytes) once this decision is known.  If that level's rows are not in
-                    // shared memory, start them towards L1 now: an L2 round trip (~1 k cycles under load, twice per sample) leaves the serial
-                    // chain indices -> tiles -> GRU -> sampler -> indices.
-                    if (b + 2 < 8 && ch == 0) {
-                        const int i2 = (1 << (b + 2)) | (val << 1);
-                        if (!(b + 2 < 3 || (b + 2 < 6 && i2 + 1 < fcw_nodes))) {
-                            const char *r2 = reinterpret_cast<const char *>(P.fcw + (size_t)i2 * FCW_ROW);
-                            asm volatile("prefetch.global.L1 [%0];" ::"l"(r2));
-                            asm volatile("prefetch.global.L1 [%0];" ::"l"(r2 + 128));
-                            asm volatile("prefetch.global.L1 [%0];" ::"l"(r2 + 256));
-                            asm volatile("prefetch.global.L1 [%0];" ::"l"(r2 + 2 * FCW_ROW * 4 - 4));
-                        }
-                    }
-#endif
                 }
                 int exc = val;
                 float pcm;

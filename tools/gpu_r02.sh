@@ -1,6 +1,6 @@
 #!/bin/bash
 # One GPU session of round 2: parity tests (incl. the at-size pins), smoke, bench lines of all three workloads, CPU arm,
-# variant sweep, ncu launch list + full capture of the per-sample kernel.   usage: tools/gpu_r02.sh <tag> [skip-tests] [skip-ncu]
+# ncu launch list + full capture of the per-sample kernel.   usage: tools/gpu_r02.sh <tag> [skip-tests] [skip-ncu]
 TAG=${1:-r02}
 mkdir -p gpurun_out
 set -x
@@ -22,7 +22,6 @@ d=json.loads(open("gpurun_out/bench_${W}_${TAG}.json").read().strip().splitlines
 print("$W", {k:d[k] for k in ("value","ms_per_step")}, "e2e", d["e2e"]["value"], "roofline frac", d["roofline"]["frac"], "cpu", d.get("cpu_baseline",{}).get("value"), d.get("cpu_baseline",{}).get("one_core_value"))
 PY
 done
-timeout 900 python tools/sweep.py run 2>&1 | tee gpurun_out/sweep_${TAG}.txt
 timeout 600 python tools/probe_bench.py 14 256 1024 4096 4736 2>&1 | tail -6 | tee gpurun_out/probe_${TAG}.txt
 if [ "$3" != "skip-ncu" ]; then
 # every launch with its device time (cold-cache, serialised: compare shares)
